@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - cells x genes / s through the smooth block + HMM (BASELINE.json metric).
 
-    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the workload: run() steps 4, 8-12, 14 (fused smooth block) followed by
 step 17 (per-cell Viterbi) on a synthetic depth-normalised matrix; c4 adds apply_median_filtering.
@@ -22,7 +22,8 @@ region; `roofline` = the dominant kernel against measured HBM bandwidth; `cpu_ba
 cores over a bounded sample.
 
 `--impl reference` times the CPU restatement of the reference's algorithm (oracle/; the reference itself is interpreted
-R: when `Rscript` and the reference's R sources are reachable the arm source()s them instead, kind "reference-R") with
+R: when `Rscript` is on the PATH and ICNV_REFERENCE_R_DIR names the reference's R/ directory the arm source()s its
+sources instead, kind "reference-R") with
 all host threads on a bounded sample of the same workload.
 """
 from __future__ import annotations
@@ -372,14 +373,14 @@ def cpu_step_fn(cfg, X, cs, cl, ref_local, lists, nt):
 
 
 def rscript_reference(args, cfg, G, C_total, seed):
-    """The real reference, when the box has it: `Rscript` plus the reference's R/ directory (ICNV_REFERENCE_R_DIR, or
-    /root/reference/R in the build container).  tools/reference_arm.R source()s the hot-path functions and times them on
-    a sample written to a temp file.  Returns the JSON dict it printed, or None (the usual case: no R in this image)."""
+    """The real reference, when the caller provides it: `Rscript` plus the reference's R/ directory named by
+    ICNV_REFERENCE_R_DIR.  tools/reference_arm.R source()s the hot-path functions and times them on a sample written to
+    a temp file.  Returns the JSON dict it printed, or None (no Rscript, or ICNV_REFERENCE_R_DIR unset)."""
     import shutil
     rs = shutil.which("Rscript")
-    rdir = os.environ.get("ICNV_REFERENCE_R_DIR") or "/root/reference/R"
+    rdir = os.environ.get("ICNV_REFERENCE_R_DIR")
     script = os.path.join(ROOT, "tools", "reference_arm.R")
-    if not rs or not os.path.isdir(rdir) or not os.path.exists(script):
+    if not rs or not rdir or not os.path.isdir(rdir) or not os.path.exists(script):
         return None
     try:
         n = min(C_total, 200)   # interpreted R: ~0.3-0.5 s per cell for the Viterbi alone
@@ -469,6 +470,37 @@ def cpu_baseline(args, cfg, G, C_total, seed):
 
 
 # ---- GPU arm --------------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20        # --dump-outputs writes at most this many bytes of array data
+
+
+def dump_outputs(out_dir, cells, C_total, G, Y, states, F, world, rank):
+    """--dump-outputs: what the timed path computed in its last step - the smoothed matrix, the HMM states and (c4) the
+    median-filtered matrix - for a sample of cells drawn with a fixed seed, rows in global cell order, so that two builds
+    can be compared output for output.  Every rank contributes the sampled cells it holds; rank 0 writes."""
+    import torch
+    import torch.distributed as dist
+    per_cell = 8 + G * (8 + 4 + (8 if F is not None else 0))
+    n = min(C_total, max(1, DUMP_BYTES // per_cell))
+    pick = np.sort(np.random.default_rng(SEED0).choice(C_total, n, replace=False))
+    rows = np.flatnonzero(np.isin(cells, pick))
+    idx = torch.as_tensor(rows, device=Y.device)
+    part = {"cells": np.asarray(cells)[rows].astype(np.float64), "smoothed": Y[idx].cpu().numpy(),
+            "states": states[idx].cpu().numpy().astype(np.float32)}
+    if F is not None:
+        part["median_filtered"] = F[idx].cpu().numpy()
+    parts = [part]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+    if rank != 0:
+        return
+    out = {k: np.concatenate([p[k] for p in parts]) for k in part}
+    order = np.argsort(out["cells"], kind="stable")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[order])
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS))
@@ -482,7 +514,12 @@ def main():
     ap.add_argument("--ref-sample-cells", type=int, default=512)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's outputs for a fixed, seeded sample of cells to DIR/*.npy "
+                         "(GPU arm only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; --impl reference has none to write")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     world_env = int(os.environ.get("WORLD_SIZE", "1"))
@@ -596,6 +633,8 @@ def main():
             raise SystemExit("non-finite / underflow flag raised during the benchmark")
     smin, smax = int(states.min().item()), int(states.max().item())
     assert 1 <= smin and smax <= (6 if cfg["hmm"] == "i6" else 3), (smin, smax)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cells, C_total, G, Y, states, Fext[:C_local] if cfg["median_filter"] else None, world, rank)
 
     # ---- end to end through the host-facing API from PAGEABLE host memory, copies inside the timed region ----
     e2e = None

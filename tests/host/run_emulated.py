@@ -28,7 +28,8 @@ assert _lib._lib is None
 
 full = "--full" in sys.argv
 extra = [a for a in sys.argv[1:] if a != "--full"]
-NEVER = ["test_device_resident_states_from_the_viterbi_kernel_to_regions", "test_full_size_round_trip_and_run_count"]
+NEVER = ["test_device_resident_states_from_the_viterbi_kernel_to_regions", "test_full_size_round_trip_and_run_count",
+         "test_engine_slab_pipelined_host_path_is_bit_identical"]
 SLOW = ["test_multi_slab_host_pipeline_and_fused_call", "test_oligodendroglioma_hmm_cells_and_samples",
         "test_oligodendroglioma_smooth_block_two_ref_groups", "test_viterbi_modes_agree_with_oracle_at_scale"]
 files = ["test_gpu_ops_mirror.py", "test_gpu_parity.py", "test_gpu_widen_denoise.py", "test_gpu_widen_elementwise.py",

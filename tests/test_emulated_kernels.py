@@ -75,17 +75,20 @@ def test_engine_and_multi_rank_path_under_the_host_emulation(world):
 
 @pytest.mark.skipif(shutil.which("g++") is None and not os.path.exists("/usr/bin/g++"), reason="no host compiler")
 @pytest.mark.parametrize("world,config", [(1, "c3"), (2, "c3"), (2, "c4")])
-def test_bench_script_reaches_its_json_line_under_the_host_emulation(world, config):
-    """bench.py itself (workload, warm-up + timed loop, e2e through the host ABI, max over ranks, JSON assembly) at a toy
-    size on the CPU, for 1 rank and for 2 ranks launched the way torchrun launches them.  The numbers are meaningless
-    (emulation, wall clock); the contract keys and the multi-rank control flow are what is checked."""
+def test_bench_script_reaches_its_json_line_under_the_host_emulation(world, config, tmp_path):
+    """bench.py itself (workload, warm-up + timed loop, e2e through the host ABI, max over ranks, JSON assembly, the
+    --dump-outputs files) at a toy size on the CPU, for 1 rank and for 2 ranks launched the way torchrun launches them.
+    The numbers are meaningless (emulation, wall clock); the contract keys and the multi-rank control flow are what is
+    checked."""
     import json
     import socket
     s = socket.socket()
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]
     s.close()
-    args = ["--gpus", str(world), "--config", config, "--steps", "2", "--warmup", "3", "--ref-sample-cells", "16"] + \
+    dump = tmp_path / "outputs"
+    args = ["--gpus", str(world), "--config", config, "--steps", "2", "--warmup", "3", "--ref-sample-cells", "16",
+            "--dump-outputs", str(dump)] + \
         (["--cells", "64", "--genes", "1100"] if config == "c3" else ["--cells", "700", "--genes", "260"])
     procs = []
     for r in range(world):
@@ -108,6 +111,31 @@ def test_bench_script_reaches_its_json_line_under_the_host_emulation(world, conf
     assert {"value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step"} <= set(j["e2e"]) and j["e2e"]["h2d_bytes_per_step"] > 0
     if world == 1:
         assert {"value", "unit", "cores", "kind", "sample"} <= set(j["cpu_baseline"])
+    import numpy as np
+    got = {f.name: np.load(f) for f in dump.iterdir()}
+    assert set(got) == {"cells.npy", "smoothed.npy", "states.npy"} | ({"median_filtered.npy"} if config == "c4" else set())
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    n, G = j["config"]["cells"], j["config"]["genes"]
+    assert np.array_equal(got["cells.npy"], np.arange(n))         # the toy sizes fit the dump budget whole
+    assert all(v.shape == (n, G) for k, v in got.items() if k != "cells.npy")
+    # every row against the oracle on the seeded workload at its global cell index (also checks the 2-rank gather order);
+    # the HMM and the median filter are re-run on the dumped smoothed matrix, so only their own arithmetic is compared
+    import bench
+    from oracle import oracle as orc
+    seed = bench.SEED0 + bench.CONFIGS[config]["index"]
+    cs, cl = bench.chr_layout(G)
+    refs = bench.ref_groups_global(n)
+    want = orc.smooth_block(orc.synth(G, cs, cl, np.arange(n), n, seed), cs, cl, refs)
+    S = np.asfortranarray(got["smoothed.npy"].T)
+    assert float(np.max(np.abs(S - want) / np.abs(want))) < 1e-11
+    if config == "c3":
+        Pi, delta, mean, sd = bench.i6_model()
+    else:
+        Pi, delta, mean, sd = bench.i3_model(*orc.mean_sd_over_cells(S, np.concatenate(refs)))
+    assert np.array_equal(got["states.npy"].T, orc.viterbi_matrix(S, cs, cl, Pi, delta, mean, sd))
+    if config == "c4":
+        lists = bench.subclusters_global(n, seed) + refs
+        assert np.allclose(got["median_filtered.npy"].T, orc.median_filter(S, cs, cl, lists, 7), rtol=0, atol=1e-15)
 
 
 def test_the_package_cannot_reach_the_emulated_library():

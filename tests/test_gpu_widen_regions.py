@@ -200,9 +200,6 @@ def test_device_resident_states_from_the_viterbi_kernel_to_regions():
         _same_regions(eng.cnv_regions(dS, cs, cl, gs, ge, cols=cells), orr.cnv_regions(S[:, cells], cs, cl, gs, ge))
 
 
-@pytest.mark.skipif(os.environ.get("ICNV_TEST_PIPELINED_HOST") != "1",
-                    reason="Engine.smooth_hmm_host was written after the last GPU session: opt-in (ICNV_TEST_PIPELINED_HOST=1) "
-                           "until its three-stream path has run on a GPU once")
 def test_engine_slab_pipelined_host_path_is_bit_identical():
     """Engine.smooth_hmm_host (reference columns first, then H2D / pass 2 + Viterbi / D2H overlapped over cell slabs on three
     streams, pinned host tensors) against smooth_block + viterbi on the uploaded matrix: identical bits."""

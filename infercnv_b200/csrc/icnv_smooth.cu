@@ -1211,7 +1211,9 @@ __global__ void __launch_bounds__(NT, MINB) cell_pipeline4_kernel(const Cell4Par
     double *cand = tails + 2 * NW;
     Red<NW> &red = *reinterpret_cast<Red<NW> *>(cand + CAND_MAX + 2);
     unsigned long long *bar = reinterpret_cast<unsigned long long *>(&red + 1);
-    int4 *ctab = reinterpret_cast<int4 *>(bar + 2);           // [n_chunks] chunk descriptors
+    // [n_chunks] chunk descriptors, read and written as int4: 16-byte aligned (an odd h leaves `bar` 8 bytes past a 16-byte
+    // boundary, the doubles in front of it being nb + h + 2 + 2 K + 2 NW + CAND_MAX + 2 with nb even)
+    int4 *ctab = reinterpret_cast<int4 *>(bar + 2 + (p.h & 1));
     int *hist = reinterpret_cast<int *>(ctab + p.n_chunks);   // NB bins, zero between cells
     int *hres = hist + NB;
     int *wcnt = hres + 8;                                     // [2][NW]
@@ -1586,6 +1588,10 @@ static int build_segments(int64_t G, const int32_t *chr_start, const int32_t *ch
     }
     if (K > 0 && chr_start[0] != 0) return -1;
     if (covered != G) return -1;
+    // every non-empty chromosome needs a thread of its own, whatever the segment length
+    int nonempty = 0;
+    for (int k = 0; k < K; ++k) nonempty += chr_len[k] > 0 ? 1 : 0;
+    if (nonempty > NT) return 0;
     // L odd: adjacent threads then start an odd number of 8-byte words apart, so the strided
     // 64-bit shared-memory accesses are bank-conflict free within a half-warp.
     for (int L = 1; L < lmax; L += 2) {
@@ -1698,6 +1704,23 @@ int icnv_dev_bounds_from_means_f64(const double *means, int64_t G, int n_grp, do
     return ICNV_OK;
 }
 
+// the compiled kernel the last icnv_dev_cell_pipeline_f64 call launched (host side; read by icnv_debug_cell_launch)
+static int g_cell_launch[8];
+
+static void record_cell_launch(int version, int nt, int padq, int lfix, int minb, int seg_len, int64_t grid, int64_t resident) {
+    const int v[8] = {version, nt, padq, lfix, minb, seg_len, (int)grid, (int)resident};
+    memcpy(g_cell_launch, v, sizeof(v));
+}
+
+// test hook, not part of the public header: {version (3 / 4), threads, padded Q, fixed slice length, min CTAs per SM,
+// segment length, grid, CTAs the launcher lets run at once (the grid of a launch with enough cells)} of the last
+// cell-pipeline launch
+ICNV_API int icnv_debug_cell_launch(int *out) {
+    if (!out) return set_error(ICNV_E_BAD_ARG, "icnv_debug_cell_launch: bad argument");
+    memcpy(out, g_cell_launch, sizeof(g_cell_launch));
+    return ICNV_OK;
+}
+
 ICNV_API int icnv_debug_stats(unsigned long long *out4, int reset) {
     ICNV_REQUIRE_READY();
     ICNV_CUDA(cudaDeviceSynchronize());
@@ -1752,14 +1775,19 @@ int icnv_dev_cell_pipeline_f64(const double *X, int64_t G, int64_t ldx, const in
         int nt3 = (G <= 2048) ? 256 : (G <= 6144 ? 512 : 1024);
         if (ctx().opt_cell_nt) nt3 = ctx().opt_cell_nt;
         if (nt3 != 256 && nt3 != 512 && nt3 != 1024) nt3 = 1024;
+        int L3 = want_v2 ? 0 : build_segments(G, chr_start, chr_len, K, nt3, 1 << 20, segs);
+        if (L3 < 0) return set_error(ICNV_E_BAD_ARG, "chromosome ranges must tile [0, G) contiguously");
+        // more chromosomes than the gene count's thread count: the next larger CTA (one thread per chromosome at least)
+        while (L3 == 0 && !ctx().opt_cell_nt && nt3 < 1024) {
+            nt3 *= 2;
+            L3 = build_segments(G, chr_start, chr_len, K, nt3, 1 << 20, segs);
+        }
         const int NW3 = nt3 / 32;
         const size_t red3 = (nt3 == 256) ? sizeof(Red<8>) : (nt3 == 512 ? sizeof(Red<16>) : sizeof(Red<32>));
         // padded-Q layout (see the kernel) whenever it fits; ICNV_CELL_PADQ=0 keeps the ping-pong layout (A/B switch)
         int padq = 1;
         padq = padq && ctx().opt_cell_padq != 0;
         const int q_elems = (int)(((int64_t)G + (int64_t)K * (2 * h + 2) + 1) & ~(int64_t)1);
-        int L3 = want_v2 ? 0 : build_segments(G, chr_start, chr_len, K, nt3, 1 << 20, segs);
-        if (L3 < 0) return set_error(ICNV_E_BAD_ARG, "chromosome ranges must tile [0, G) contiguously");
         const int ipad = (L3 + 2) & ~1;   // front pad of the reciprocal-denominator table: >= the longest slice, even
         auto smem_for = [&](bool pq) {
             const size_t cols = pq ? (size_t)q_elems + (size_t)s_elems + (size_t)ipad
@@ -1786,6 +1814,7 @@ int icnv_dev_cell_pipeline_f64(const double *X, int64_t G, int64_t ldx, const in
             // fully unrolled slice loops for the segment length of the 10 000-gene configurations (ICNV_CELL_LFIX=0: generic)
             int lfix = (padq && nt3 == 1024 && L3 == 11) ? 11 : 0;
             if (ctx().opt_cell_lfix == 0) lfix = 0;
+            record_cell_launch(3, nt3, padq, lfix, 1, L3, grid3, c.sm_count);
             if (lfix == 11)
                 rc3 = launch3(cell_pipeline3_kernel<1024, true, 11>);
             else if (padq)
@@ -1838,6 +1867,7 @@ int icnv_dev_cell_pipeline_f64(const double *X, int64_t G, int64_t ldx, const in
             const int nw = nt / 32;
             const size_t red = (nt == 256) ? sizeof(Red<8>) : (nt == 512 ? sizeof(Red<16>) : sizeof(Red<32>));
             return 128 * 24 + sizeof(double) * ((size_t)nb + (size_t)(h + 2) + 2 * (size_t)K + 2 * (size_t)nw + CAND_MAX + 2) + red + 16 +
+                   sizeof(double) * (size_t)(h & 1) +   // alignment of the chunk table (see the kernel)
                    sizeof(int) * (1024 + 8 + 2 * (size_t)nw + 2 + 32) + sizeof(Chr4) * ((size_t)K + 1) + sizeof(int4) * (size_t)nch + 16;
         };
         const size_t sm_total = 228 * 1024;     // shared memory of an SM; every resident CTA also reserves 1 KB
@@ -1857,6 +1887,12 @@ int icnv_dev_cell_pipeline_f64(const double *X, int64_t G, int64_t ldx, const in
         }
         int L4 = build_segments(G, chr_start, chr_len, K, nt4, 1 << 20, segs);
         if (L4 < 0) return set_error(ICNV_E_BAD_ARG, "chromosome ranges must tile [0, G) contiguously");
+        // more chromosomes than threads: the next larger CTA, with as many CTAs per SM as its shared memory allows
+        while (L4 == 0 && !c.opt_cell_nt && nt4 < 1024) {
+            nt4 *= 2;
+            minb = std::max(1, std::min(nt4 == 512 ? 2 : 1, (int)(sm_total / (smem4(nt4) + 1024))));
+            L4 = build_segments(G, chr_start, chr_len, K, nt4, 1 << 20, segs);
+        }
         const size_t smem = smem4(nt4);
         if (L4 > 0 && smem <= (size_t)c.smem_optin) {
             const size_t off_chr = sizeof(Seg) * 1024, off_chunks = (off_chr + sizeof(Chr4) * ((size_t)K + 1) + 15) & ~(size_t)15;
@@ -1876,31 +1912,36 @@ int icnv_dev_cell_pipeline_f64(const double *X, int64_t G, int64_t ldx, const in
             q.apply_log = apply_log; q.lo1 = lo1; q.hi1 = hi1; q.mid1 = mid1; q.threshold = threshold;
             q.window = window; q.h = h; q.center = center; q.lo2 = lo2; q.hi2 = hi2; q.mid2 = mid2;
             q.apply_exp2 = apply_exp2; q.err_flag = err_flag; q.K = K; q.nb = nb; q.n_chunks = nch;
-            auto launch4 = [&](auto kern) -> int {
+            auto launch4 = [&](auto kern, int kminb, int klfix) -> int {
                 ICNV_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
                 int per_sm = 1;
                 ICNV_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nt4, smem));
-                const int64_t grid = std::min<int64_t>(n_cols, (int64_t)c.sm_count * std::max(per_sm, 1));
+                const int64_t resident = (int64_t)c.sm_count * std::max(per_sm, 1);
+                const int64_t grid = std::min<int64_t>(n_cols, resident);
+                record_cell_launch(4, nt4, 0, klfix, kminb, L4, grid, resident);
                 kern<<<(unsigned)grid, nt4, smem, st>>>(q);
                 return ICNV_OK;
             };
             int rc4;
             // the slice length of the 10 000-gene / 20 000-gene layouts (21 genes per thread) gets fully unrolled scan passes
             const bool fix21 = L4 == 21 && c.opt_cell_lfix != 0;
-            if (nt4 == 256) rc4 = (minb >= 4) ? launch4(cell_pipeline4_kernel<256, 4, 1024, 0>) : launch4(cell_pipeline4_kernel<256, 1, 1024, 0>);
-            else if (nt4 == 512 && minb >= 2) rc4 = fix21 ? launch4(cell_pipeline4_kernel<512, 2, 1024, 21>) : launch4(cell_pipeline4_kernel<512, 2, 1024, 0>);
-            else if (nt4 == 512) rc4 = launch4(cell_pipeline4_kernel<512, 1, 1024, 0>);
-            else rc4 = fix21 ? launch4(cell_pipeline4_kernel<1024, 1, 1024, 21>) : launch4(cell_pipeline4_kernel<1024, 1, 1024, 0>);
+            if (nt4 == 256) rc4 = (minb >= 4) ? launch4(cell_pipeline4_kernel<256, 4, 1024, 0>, 4, 0) : launch4(cell_pipeline4_kernel<256, 1, 1024, 0>, 1, 0);
+            else if (nt4 == 512 && minb >= 2) rc4 = fix21 ? launch4(cell_pipeline4_kernel<512, 2, 1024, 21>, 2, 21) : launch4(cell_pipeline4_kernel<512, 2, 1024, 0>, 2, 0);
+            else if (nt4 == 512) rc4 = launch4(cell_pipeline4_kernel<512, 1, 1024, 0>, 1, 0);
+            else rc4 = fix21 ? launch4(cell_pipeline4_kernel<1024, 1, 1024, 21>, 1, 21) : launch4(cell_pipeline4_kernel<1024, 1, 1024, 0>, 1, 0);
             if (rc4) return rc4;
             ICNV_CHECK_LAUNCH("cell_pipeline4_kernel");
             return ICNV_OK;
         }
-        if (!(L4 > 0))
-            return set_error(ICNV_E_UNSUPPORTED, "G = %lld genes in K = %d chromosomes need more than 1024 per-thread slices", (long long)G, K);
+        if (!(L4 > 0)) {
+            int nonempty = 0;
+            for (int k = 0; k < K; ++k) nonempty += chr_len[k] > 0 ? 1 : 0;
+            return set_error(ICNV_E_UNSUPPORTED, "%d non-empty chromosomes need a thread each, more than the %d threads of a CTA",
+                             nonempty, nt4);
+        }
+        return set_error(ICNV_E_UNSUPPORTED, "G = %lld genes in %d chromosomes, window %d: a cell's padded column needs %lld B of "
+                         "shared memory, more than the %d B a CTA can have", (long long)G, K, window, (long long)smem, c.smem_optin);
     }
-
-    return set_error(ICNV_E_UNSUPPORTED, "G = %lld genes, window %d: the cell's padded column (%lld doubles) does not fit the %d B of "
-                     "shared memory a CTA can have", (long long)G, window, (long long)(G + (int64_t)K * (2 * h + 3)), c.smem_optin);
 }
 
 }  // extern "C"
